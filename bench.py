@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Benchmark of the TAPIR hot path (driver contract: see the task brief / DESIGN.md section 6).
+"""Benchmark of the TAPIR hot path (DESIGN.md section 6).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one full inference pass  get_feature_grids + get_query_features +
 estimate_trajectories (+ the per-level mean of forward)  over one synthetic clip.
@@ -18,6 +18,10 @@ rules (warm-up >= 3, CUDA events, max over ranks, L2 flushed between steps, own 
   sub_records.c5_hires   configs[4]  1024x1024x64, 8192 queries, three refinement levels
 and `roofline_named` holds the per-kernel roofline objects of the two kernels BASELINE.json's
 north star names (global cost volume, local correlation) next to `roofline` (largest share).
+
+--dump-outputs DIR writes what the last timed headline step returned as .npy files; inputs and
+weights come from fixed seeds, so two builds run with the same arguments can be compared output
+for output.
 """
 import argparse
 import ctypes
@@ -193,15 +197,17 @@ class Runner:
 
   def timed(self, fn, steps):
     """K steps inside one barrier+sync bracket; per-step CUDA events; L2 flushed between steps.
-    Returns (ms per step = max over ranks of the per-rank mean, clocks window)."""
+    Returns (ms per step = max over ranks of the per-rank mean, clocks window, what the last
+    step's fn() returned)."""
     evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
            for _ in range(steps)]
     self.barrier()
     t0 = time.time()
     for a, b in evs:
+      out = None  # release the previous step's outputs before the next step, as a caller would
       self.flush.zero_()
       a.record()
-      fn()
+      out = fn()
       b.record()
     self.barrier()
     t1 = time.time()
@@ -210,7 +216,7 @@ class Runner:
     if self.world > 1:
       self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
     clocks = self.sampler.window(t0, t1) if self.rank == 0 else None
-    return t.item() / steps, clocks
+    return t.item() / steps, clocks, out
 
   def profile(self, fn, reps=2):
     """Per-kernel device time: CUDA events around every launch of the library on its stream."""
@@ -265,8 +271,41 @@ def roofline_hbm(name, v, peaks):
               launches=v['launches'], avg_launch_ms=round(v['ms'] / v['launches'], 4))
 
 
-def run_offline_workload(R, name, steps, warmup, with_profile=True, legs=('device', 'e2e', 'e2e_u8')):
-  """One offline workload (c2 / c4 / c5) -> record dict (rank 0) or None."""
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, out, num_queries, world, rank):
+  """Writes what one call of the timed path returned as float32 `<key>.npy` files: `tracks`,
+  `occlusion`, `expected_dist` ([1, N, T(, 2)]) and, where the call returns them, the
+  per-iteration `unrefined_*` lists stacked on a new leading axis.  Query shards are gathered
+  first (a collective when world > 1; rank 0 writes).  Above DUMP_LIMIT bytes in all, every array
+  keeps the same seeded sample of query points, whose indices go to `query_index.npy`."""
+  import numpy as np  # pylint: disable=g-import-not-at-top
+  from tapnet_b200 import distributed as tdist  # pylint: disable=g-import-not-at-top
+  arrays = {}
+  for k, v in out.items():
+    qaxis = 2 if isinstance(v, (list, tuple)) else 1
+    t = torch.stack(list(v)) if qaxis == 2 else v
+    if world > 1:
+      t = tdist.gather_queries(t, num_queries, qaxis)
+    arrays[k] = (t.float().cpu().numpy(), qaxis)
+  if rank != 0:
+    return
+  total = sum(a.nbytes for a, _ in arrays.values())
+  if total > DUMP_LIMIT:
+    keep = DUMP_LIMIT // (total // num_queries + 8)  # + 8 bytes per query for query_index
+    idx = np.sort(np.random.default_rng(0).choice(num_queries, keep, replace=False))
+    arrays = {k: (np.take(a, idx, axis=qaxis), qaxis) for k, (a, qaxis) in arrays.items()}
+    arrays['query_index'] = (idx.astype(np.float64), 0)
+  os.makedirs(out_dir, exist_ok=True)
+  for k, (a, _) in arrays.items():
+    np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
+def run_offline_workload(R, name, steps, warmup, with_profile=True, legs=('device', 'e2e', 'e2e_u8'),
+                         dump_dir=None):
+  """One offline workload (c2 / c4 / c5) -> record dict (rank 0) or None.  With dump_dir, the
+  outputs of the last timed device step are written there (dump_outputs)."""
   from tapnet_b200 import distributed as tdist
   wl = WORKLOADS[name]
   world, rank, dev, model = R.world, R.rank, R.dev, R.model
@@ -304,21 +343,24 @@ def run_offline_workload(R, name, steps, warmup, with_profile=True, legs=('devic
     step_device()
   R.barrier()
   launches0 = R.lib.tapir_launch_count()
-  ms_step, clocks = R.timed(step_device, steps)
+  ms_step, clocks, last = R.timed(step_device, steps)
   launches = (R.lib.tapir_launch_count() - launches0) // max(steps, 1)
+  if dump_dir:
+    dump_outputs(dump_dir, last, N, world, rank)
+  del last
   d2h = int(sum(t.numel() * 4 for t in out_pin.values()))
   e2e = e2e_u8 = None
   if 'e2e' in legs and video_pin is not None:
     f = make_e2e(video_pin)
     f()
-    ms, _ = R.timed(f, steps)
+    ms, _, _ = R.timed(f, steps)
     e2e = dict(value=round(N * T / (ms * 1e-3), 1), unit=UNIT, ms_per_step=round(ms, 3),
                h2d_bytes_per_step=int(video_h.numel() * 4 + queries_h.numel() * 4),
                d2h_bytes_per_step=d2h, frames='float32 [-1,1]')
   if 'e2e_u8' in legs:
     f = make_e2e(frames_u8_pin)
     f()
-    ms, _ = R.timed(f, steps)
+    ms, _, _ = R.timed(f, steps)
     e2e_u8 = dict(value=round(N * T / (ms * 1e-3), 1), unit=UNIT, ms_per_step=round(ms, 3),
                   h2d_bytes_per_step=int(video_h.numel() + queries_h.numel() * 4),
                   d2h_bytes_per_step=d2h,
@@ -438,7 +480,7 @@ def run_c3_stream(R):
 def run_ours(args):
   R = Runner(args)
   world, rank = R.world, R.rank
-  main = run_offline_workload(R, args.workload, args.steps, args.warmup)
+  main = run_offline_workload(R, args.workload, args.steps, args.warmup, dump_dir=args.dump_outputs)
   sub = {}
   if not args.no_sub and args.workload == 'c2':
     sub_steps = max(2, min(args.steps, 5))
@@ -522,23 +564,21 @@ def run_ours(args):
 
 
 def _load_reference_module():
-  """The UNMODIFIED reference torch path, if it can be imported on this box: `baseline/_ref`
-  (pip --target install of /root/reference made in the build container, git-ignored, travels
-  with the snapshot) or /root/reference itself (build container only).  Layout-only shims for
-  its two absent dependencies (einshape, dm-tree) come from oracle/shims.  Returns the module
-  `tapnet.torch.tapir_model` or None."""
-  shims = os.path.join(ROOT, 'oracle', 'shims')
-  for root in (os.path.join(ROOT, 'baseline', '_ref'), '/root/reference'):
-    if os.path.isfile(os.path.join(root, 'tapnet', 'torch', 'tapir_model.py')):
-      for p in (root, shims):
-        if p not in sys.path:
-          sys.path.insert(0, p)
-      try:
-        from tapnet.torch import tapir_model as ref  # pylint: disable=g-import-not-at-top
-        return ref, root
-      except Exception:  # pylint: disable=broad-except
-        continue
-  return None, None
+  """The UNMODIFIED reference torch path, if it is installed in the tree: `baseline/_ref`
+  (a git-ignored `pip install --target baseline/_ref` of the original tapnet package).
+  Layout-only shims for its two absent dependencies (einshape, dm-tree) come from oracle/shims.
+  Returns (the module `tapnet.torch.tapir_model`, its root) or (None, None)."""
+  root = os.path.join(ROOT, 'baseline', '_ref')
+  if not os.path.isfile(os.path.join(root, 'tapnet', 'torch', 'tapir_model.py')):
+    return None, None
+  for p in (root, os.path.join(ROOT, 'oracle', 'shims')):
+    if p not in sys.path:
+      sys.path.insert(0, p)
+  try:
+    from tapnet.torch import tapir_model as ref  # pylint: disable=g-import-not-at-top
+    return ref, root
+  except Exception:  # pylint: disable=broad-except
+    return None, None
 
 
 SAMPLE_FRAMES, SAMPLE_QUERIES = 4, 16
@@ -690,7 +730,9 @@ def run_reference(args):
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--gpus', type=int, default=1)
-  ap.add_argument('--steps', type=int, default=20)
+  ap.add_argument('--steps', type=int, default=20,
+                  help='timed steps of each leg of the headline workload (sub-records keep their '
+                       'own short budgets)')
   ap.add_argument('--warmup', type=int, default=3)
   ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
   ap.add_argument('--precision', default='bf16x3', choices=['bf16', 'bf16x3', 'bf16x6'])
@@ -698,7 +740,11 @@ def main():
   ap.add_argument('--no-sub', action='store_true', help='skip the c4 / c3 / c5 sub-records')
   ap.add_argument('--workload', default='c2', choices=['c2', 'c4', 'c5'],
                   help='headline workload: c2 = driver contract (default)')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write the outputs of the last timed headline step to DIR/<name>.npy')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
   if args.impl == 'reference':
     run_reference(args)
   else:

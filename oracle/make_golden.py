@@ -132,11 +132,35 @@ def run_case(name):
   return out
 
 
+# constructor keywords whose state_dict layout tests/test_schema.py pins
+SCHEMA_KWARGS = {'pl1': dict(pyramid_level=1), 'pl0_noextra': dict(pyramid_level=0, extra_convs=False)}
+# frame sizes whose generate_default_resolutions(size, (256, 256)) tests/test_host_logic.py pins
+RESOLUTION_SIZES = [(256, 256), (240, 240), (480, 480), (480, 640), (360, 640), (512, 512),
+                    (720, 1280), (1024, 1024), (1080, 1920), (264, 264), (250, 500), (2048, 1024)]
+
+
+def run_interface():
+  """The reference's host-side interface, no compute: state_dict key order and shapes per
+  constructor, and the refinement resolutions it picks per frame size (utils.py:275-317)."""
+  import contextlib  # pylint: disable=g-import-not-at-top
+  import io  # pylint: disable=g-import-not-at-top
+  ref = reference_loader.load()
+  from tapnet.torch import utils as ref_utils  # pylint: disable=g-import-not-at-top
+  schema = {k: [[name, list(v.shape)] for name, v in ref.TAPIR(**kw).state_dict().items()]
+            for k, kw in SCHEMA_KWARGS.items()}
+  with contextlib.redirect_stdout(io.StringIO()):   # the non-multiple-of-8 warning
+    res = [[list(hw), [[int(v) for v in r] for r in ref_utils.generate_default_resolutions(hw, (256, 256))]]
+           for hw in RESOLUTION_SIZES]
+  meta = dict(name='reference_interface', schema=schema, schema_kwargs=SCHEMA_KWARGS,
+              default_resolutions=res, torch=torch.__version__)
+  return {'meta': np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)}
+
+
 def main():
   import sys  # pylint: disable=g-import-not-at-top
   os.makedirs(GOLDEN_DIR, exist_ok=True)
-  for name in (sys.argv[1:] or CASES):
-    out = run_case(name)
+  for name in (sys.argv[1:] or ['reference_interface', *CASES]):
+    out = run_interface() if name == 'reference_interface' else run_case(name)
     path = os.path.join(GOLDEN_DIR, name + '.npz')
     np.savez_compressed(path, **out)
     print(name, os.path.getsize(path), 'bytes')

@@ -1,5 +1,5 @@
 """bench.py's CPU legs: the reference arm must be the UNMODIFIED reference whenever it is importable
-(baseline/_ref on the GPU box, /root/reference in the build container), the oracle port otherwise."""
+(installed under baseline/_ref), the oracle port otherwise."""
 import os
 import sys
 
@@ -13,8 +13,7 @@ from tapnet_b200 import synth  # noqa: E402
 
 
 def test_cpu_arm_runs_the_unmodified_reference_when_importable():
-  have_ref = any(os.path.isfile(os.path.join(r, 'tapnet', 'torch', 'tapir_model.py'))
-                 for r in (os.path.join(ROOT, 'baseline', '_ref'), '/root/reference'))
+  have_ref = os.path.isfile(os.path.join(ROOT, 'baseline', '_ref', 'tapnet', 'torch', 'tapir_model.py'))
   wl = dict(bench.WORKLOADS['c2'], frames=6)
   video = synth.make_video(6)
   queries = synth.make_queries(32, 6)
@@ -28,6 +27,34 @@ def test_cpu_arm_runs_the_unmodified_reference_when_importable():
   d = arm.describe(sec)
   assert sec > 0 and d['kind'] == arm.kind and d['unit'] == bench.UNIT
   assert abs(d['value'] - 32 * 6 / sec) < 1e-6 * d['value'] + 0.1
+
+
+def test_dump_outputs_writes_float32_and_samples_queries_above_the_limit(tmp_path, monkeypatch):
+  import numpy as np
+  N, T = 40, 6
+  g = torch.Generator().manual_seed(0)
+  out = dict(tracks=torch.randn(1, N, T, 2, generator=g), occlusion=torch.randn(1, N, T, generator=g),
+             unrefined_tracks=[torch.randn(1, N, T, 2, generator=g) for _ in range(3)])
+  bench.dump_outputs(str(tmp_path / 'all'), out, N, 1, 0)
+  got = {k: np.load(tmp_path / 'all' / f'{k}.npy') for k in out}
+  assert sorted(os.listdir(tmp_path / 'all')) == sorted(f'{k}.npy' for k in out)
+  assert all(a.dtype == np.float32 for a in got.values())
+  np.testing.assert_array_equal(got['tracks'], out['tracks'].numpy())
+  np.testing.assert_array_equal(got['unrefined_tracks'], torch.stack(out['unrefined_tracks']).numpy())
+  limit = 4096
+  monkeypatch.setattr(bench, 'DUMP_LIMIT', limit)
+  for run in ('a', 'b'):
+    bench.dump_outputs(str(tmp_path / run), out, N, 1, 0)
+  files = sorted(os.listdir(tmp_path / 'a'))
+  assert files == sorted(os.listdir(tmp_path / 'b')) and 'query_index.npy' in files
+  assert sum(os.path.getsize(tmp_path / 'a' / f) - 128 for f in files) <= limit  # 128 B .npy header
+  idx = np.load(tmp_path / 'a' / 'query_index.npy').astype(np.int64)
+  assert 0 < len(idx) < N and np.all(np.diff(idx) > 0)
+  for f in files:
+    np.testing.assert_array_equal(np.load(tmp_path / 'a' / f), np.load(tmp_path / 'b' / f))
+  np.testing.assert_array_equal(np.load(tmp_path / 'a' / 'tracks.npy'), got['tracks'][:, idx])
+  np.testing.assert_array_equal(np.load(tmp_path / 'a' / 'unrefined_tracks.npy'),
+                                got['unrefined_tracks'][:, :, idx])
 
 
 def _run_reference_arm(rank, world):

@@ -68,27 +68,22 @@ def test_default_resolutions():
   assert f((1024, 1024), (256, 256)) == [(256, 256), (512, 512), (1024, 1024)]
 
 
-def test_default_resolutions_sweep_matches_reference_and_oracle():
-  """generate_default_resolutions over a sweep of frame sizes: product == oracle restatement, and
-  == the reference's own function when it is mounted (utils.py:275-317)."""
+def test_default_resolutions_sweep_matches_reference_and_oracle(golden):
+  """generate_default_resolutions over a sweep of frame sizes: product == oracle restatement ==
+  the reference's own function (utils.py:275-317), whose results
+  `python -m oracle.make_golden reference_interface` stored."""
   import contextlib
   import io
-  from oracle import reference_loader
   from oracle import tapir_oracle as O
-  ref = None
-  if reference_loader.available():
-    reference_loader.load()
-    from tapnet.torch import utils as ref_utils  # pylint: disable=g-import-not-at-top
-    ref = ref_utils.generate_default_resolutions
-  sizes = [(256, 256), (240, 240), (480, 480), (480, 640), (360, 640), (512, 512), (720, 1280),
-           (1024, 1024), (1080, 1920), (264, 264), (250, 500), (2048, 1024)]
-  for hw in sizes:
+  sweep = golden('reference_interface')['meta']['default_resolutions']
+  assert len(sweep) == 12
+  for hw, ref in sweep:
+    hw = tuple(hw)
     with contextlib.redirect_stdout(io.StringIO()):   # the non-multiple-of-8 warning
       got = tapir_model.generate_default_resolutions(hw, (256, 256))
       want = O.default_resolutions(hw, (256, 256))
       assert [tuple(r) for r in got] == [tuple(r) for r in want], hw
-      if ref is not None:
-        assert [tuple(r) for r in got] == [tuple(int(v) for v in r) for r in ref(hw, (256, 256))], hw
+      assert [tuple(r) for r in got] == [tuple(r) for r in ref], hw
     assert all(r[0] % 8 == 0 and r[1] % 8 == 0 for r in got)
     assert tuple(got[0]) == (256, 256)
 

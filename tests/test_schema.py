@@ -1,6 +1,5 @@
 import pytest
 
-from oracle import reference_loader
 from tapnet_b200 import schema
 
 
@@ -12,11 +11,14 @@ def test_param_counts():
   assert len(s0) == 188
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason='reference not mounted')
 @pytest.mark.parametrize('kw', [dict(pyramid_level=1), dict(pyramid_level=0, extra_convs=False)])
-def test_schema_matches_reference_module(kw):
-  ref = reference_loader.load().TAPIR(**kw).state_dict()
+def test_schema_matches_reference_module(kw, golden):
+  """Key order and shapes of the reference module's state_dict, as stored by
+  `python -m oracle.make_golden reference_interface`."""
+  meta = golden('reference_interface')['meta']
+  (tag,) = [t for t, k in meta['schema_kwargs'].items() if k == kw]
+  ref = [(name, tuple(shape)) for name, shape in meta['schema'][tag]]
   s = schema.state_dict_schema(kw.get('pyramid_level', 1), kw.get('extra_convs', True))
-  assert list(ref.keys()) == list(s.keys())
-  for k, v in ref.items():
-    assert tuple(v.shape) == s[k], k
+  assert [name for name, _ in ref] == list(s.keys())
+  for k, shape in ref:
+    assert shape == s[k], k
